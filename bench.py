@@ -667,6 +667,19 @@ def run_c4(args, rank, world, local):
 
 
 # ----------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, model, loss):
+    """What the caller of training_step holds after the last timed step: the returned loss, the logged values and the
+    trainable parameters with their gradients (fp32; < 8 MB for ViT-B), as <name>.npy with '/' in a name written '.'."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, **{"logged." + k.replace("/", "."): v for k, v in model.logged.items()}}
+    for n, p in model.named_parameters():
+        if p.grad is not None:  # the parameters the step trains (the decoder has none without the rec term)
+            arrays["param." + n], arrays["grad." + n] = p, p.grad
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), torch.as_tensor(t).detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -682,7 +695,14 @@ def main():
     ap.add_argument("--no-kernel-rooflines", action="store_true")
     ap.add_argument("--breakdown", action="store_true", help="also report per-phase device time of the step")
     ap.add_argument("--corr-sweep", action="store_true", help="dense tensor_correlation sweep (S = 121 ... h w) and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, logged values, the trainable "
+                         "parameters and their gradients) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.corr_sweep or args.config == "c4" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the training step (--config c1|c2|c3, --impl ours)")
     cfgd = dict(CONFIGS[args.config])
     if args.batch:
         cfgd["batch"] = args.batch
@@ -777,6 +797,7 @@ def main():
         return b, ev
 
     host_ms = [0.0]
+    last_loss = [None]
 
     def run(nsteps, e2e, hb=None):
         barrier()
@@ -812,7 +833,7 @@ def main():
         else:
             t_host = time.perf_counter()
             for i in range(nsteps):
-                model.training_step(batch, i)
+                last_loss[0] = model.training_step(batch, i)
             host_ms[0] = (time.perf_counter() - t_host) * 1e3 / max(nsteps, 1)  # CPU time to ENQUEUE one step
         model.flush()  # the last step's parameter update (side stream) belongs to the timed region too
         e.record()
@@ -832,6 +853,8 @@ def main():
     host_enqueue_ms = host_ms[0]
     launches = _lib.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, last_loss[0])
     run(min(args.warmup, 3), True, host_compact)
     ms_e2e = run(args.steps, True, host_compact)
     run(min(args.warmup, 3), True, host)

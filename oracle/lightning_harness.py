@@ -8,9 +8,9 @@ What it is for
     (`modules_impl="reference"`) on the B200 (PyTorch eager, fp32 or bf16 autocast) and on the host CPU.
 
 Nothing here is product code and nothing under stego_b200/ imports it.  The reference sources are never copied
-into the repository: they are read at run time from `baseline/_ref/src` (a git-ignored verbatim copy made by
-`__graft_entry__.build()` in the build container; it travels to the GPU box with the snapshot) or, in the build
-container only, from /root/reference/src.
+into the repository: they are read at run time from the directory $STEGO_REFERENCE_SRC names (the reference's `src`)
+or from a git-ignored `baseline/_ref/src`.  oracle/make_golden.py runs the reference through this harness and stores
+what the tests compare against under tests/golden/.
 
 The stubs replace exactly the third-party names `train_segmentation.py` imports (`:1-16`):
   utils.*            -> nn, F, torch, np, os, join, plt + no-op UnsupervisedMetrics / colormaps / resize / one_hot_feats
@@ -35,12 +35,11 @@ import torch.nn.functional as F
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(_HERE)
-_CANDIDATES = [os.path.join(ROOT, "baseline", "_ref", "src"), "/root/reference/src"]
 
 
 def reference_src() -> Optional[str]:
-    for c in _CANDIDATES:
-        if os.path.isfile(os.path.join(c, "train_segmentation.py")):
+    for c in [os.environ.get("STEGO_REFERENCE_SRC", ""), os.path.join(ROOT, "baseline", "_ref", "src")]:
+        if c and os.path.isfile(os.path.join(c, "train_segmentation.py")):
             return c
     return None
 
@@ -181,8 +180,7 @@ def load_reference_segmenter(modules_impl: str = "reference"):
     The module objects are private to this call (sys.modules is restored), so both flavours can coexist."""
     src = reference_src()
     if src is None:
-        raise RuntimeError("reference sources not found (baseline/_ref/src is made by __graft_entry__.build() in the "
-                           "build container)")
+        raise RuntimeError("reference sources not found: set STEGO_REFERENCE_SRC to the reference's src directory")
     saved = {k: sys.modules.get(k) for k in _OWNED}
     saved_path = list(sys.path)
     try:
@@ -229,6 +227,29 @@ def write_random_dino_checkpoint(path: str, arch: str, seed: int = 3, perturb: b
         sd = O.perturb_vit_state(sd)
     torch.save({"teacher": sd}, path)
     return sd
+
+
+def trainable_state(n_feats: int = 384, dim: int = 70, n_classes: int = 27, seed: int = 4) -> dict:
+    """Seeded values for the nine trainable parameters (named as in LitUnsupervisedSegmenter.named_parameters()), so that a
+    stored reference run and a later run of this project start from the same state without storing it."""
+    sys.path.insert(0, _HERE)
+    import stego_oracle as O
+    sd = {"net." + k: v for k, v in O.head_random_state(n_feats, dim, seed=seed).items()}
+    g = torch.Generator().manual_seed(seed + 1)
+    b = 1.0 / dim ** 0.5
+    sd["linear_probe.weight"] = (torch.rand(n_classes, dim, 1, 1, generator=g) * 2 - 1) * b
+    sd["linear_probe.bias"] = (torch.rand(n_classes, generator=g) * 2 - 1) * b
+    sd["cluster_probe.clusters"] = torch.randn(n_classes, dim, generator=g)
+    return sd
+
+
+def load_trainable_state(model: nn.Module, sd: dict, prefix: str = "") -> None:
+    """Copy `sd` (keys as trainable_state returns them, `prefix` stripped) into the model's parameters in place."""
+    params = dict(model.named_parameters())
+    with torch.no_grad():
+        for k, v in sd.items():
+            if k.startswith(prefix):
+                params[k[len(prefix):]].copy_(v)
 
 
 def make_batch(B: int, res: int, device, seed: int = 1, n_classes: int = 27) -> dict:

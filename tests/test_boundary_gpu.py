@@ -5,9 +5,10 @@ the way the reference calls them:
   * tensor_correlation (src/modules.py:283-284);
   * DinoFeaturizer.forward with dino_feat_type "KK" and with return_class_feat (src/modules.py:98-106);
   * ClusterLookup argmax assignments: EXACT flip counts against the fp32 oracle and against an fp64 evaluation;
-  * the reference's own `LitUnsupervisedSegmenter.training_step` TEXT (src/train_segmentation.py:112-245) executed
-    over stego_b200.modules through a stub Lightning base (oracle/lightning_harness.py), compared with the same text
-    over the reference's own modules.py in PyTorch eager on the same GPU.
+  * LitUnsupervisedSegmenter.training_step compared with the reference's own (src/train_segmentation.py:112-245, over
+    its own modules.py in PyTorch eager on a B200, run by oracle/make_golden.py --gpu).
+
+The reference's outputs are stored (sampled) in tests/golden/reference_gpu.pt.
 """
 import os
 import sys
@@ -19,6 +20,15 @@ from _parity_util import fp32_strict, record, rel
 
 pytestmark = pytest.mark.gpu
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "..", "oracle"))
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_gpu.pt")
+
+
+def _rel_sampled(got, s):
+    """rel() on the elements the stored sample `s` (make_golden.sampled) holds, and the relative norm difference of
+    the whole tensors."""
+    flat = got.detach().reshape(-1).double().cpu()
+    sub = flat[s["idx"].long()] if "idx" in s else flat
+    return rel(sub, s["val"]), abs(flat.norm().item() - s["norm"]) / s["norm"]
 
 
 def _correlated(B, C, h, w, g, rank=16):
@@ -89,37 +99,34 @@ def test_tensor_correlation(cuda_dev, n, c, hw, ij):
 def test_featurizer_kk_and_class_feat(cuda_dev):
     """feat_type "KK" (keys of the last block, heads concatenated) and return_class_feat against the reference's own
     DinoFeaturizer run in PyTorch eager (fp32) on the same weights."""
-    import lightning_harness as H
-    if not H.available():
-        pytest.skip("reference sources (baseline/_ref) not present")
     import tempfile
+    import lightning_harness as H
+    import make_golden
     from stego_b200.config import make_cfg
     from stego_b200.modules import DinoFeaturizer
     fp32_strict()
-    ts = H.load_reference_segmenter("reference")
+    gold = torch.load(GOLD)
     with tempfile.TemporaryDirectory() as td:
         ck = os.path.join(td, "dino.pth")
         H.write_random_dino_checkpoint(ck, "vit_small")
-        torch.manual_seed(6)
-        img = torch.randn(2, 3, 64, 96, device=cuda_dev)
+        img = make_golden.featurizer_inputs(cuda_dev)
         for feat_type in ("KK", "feat"):
             cfg = make_cfg(dino_feat_type=feat_type, pretrained_weights=ck)
             torch.manual_seed(0)
-            ref = ts._modules.DinoFeaturizer(70, cfg).to(cuda_dev).eval()
-            torch.manual_seed(0)
             ours = DinoFeaturizer(70, cfg).to(cuda_dev).eval()
-            ours.load_state_dict(ref.state_dict())
+            H.load_trainable_state(ours, H.trainable_state(), prefix="net.")
+            want = gold[f"featurizer_{feat_type}"]
             with torch.no_grad():
-                rf, rc = ref(img)
                 of, oc = ours(img)
-                assert of.shape == rf.shape and oc.shape == rc.shape
-                assert rel(of, rf) < 1e-2, (feat_type, rel(of, rf))
-                assert rel(oc, rc) < 2e-2, (feat_type, rel(oc, rc))
+                assert tuple(of.shape) == want["feats"]["shape"] and tuple(oc.shape) == want["code"]["shape"]
+                for got, w, tol in ((of, want["feats"], 1e-2), (oc, want["code"], 2e-2)):
+                    err, norm_err = _rel_sampled(got, w)
+                    assert err < tol and norm_err < tol, (feat_type, err, norm_err)
                 if feat_type == "feat":
-                    rcls = ref(img, return_class_feat=True)
                     ocls = ours(img, return_class_feat=True)
-                    assert ocls.shape == rcls.shape == (2, 384, 1, 1)
-                    assert rel(ocls, rcls) < 1e-2
+                    assert tuple(ocls.shape) == gold["featurizer_class_feat"]["shape"] == (2, 384, 1, 1)
+                    err, norm_err = _rel_sampled(ocls, gold["featurizer_class_feat"])
+                    assert err < 1e-2 and norm_err < 1e-2, (err, norm_err)
 
 
 @pytest.mark.parametrize("B,h,w", [(2, 28, 28), (2, 40, 40), (1, 56, 56), (1, 128, 256)])
@@ -195,49 +202,38 @@ def test_eval_frame_assignments_vs_oracle(cuda_dev):
         assert flips < 200
 
 
-def test_reference_training_step_text_over_stego_modules(cuda_dev):
-    """SURVEY §7.3(9): the reference `training_step` source runs unchanged over stego_b200.modules."""
-    import lightning_harness as H
-    if not H.available():
-        pytest.skip("reference sources (baseline/_ref) not present")
+def test_training_step_vs_reference_eager(cuda_dev):
+    """Two LitUnsupervisedSegmenter.training_step calls against the reference's own two steps (PyTorch eager, fp32, on a
+    B200) from the same parameters, batch and generator state."""
     import tempfile
+    import lightning_harness as H
     from stego_b200.config import make_cfg
+    from stego_b200.segmenter import LitUnsupervisedSegmenter
+    from _parity_util import grads_of
     fp32_strict()
+    ref = torch.load(GOLD)["training_step"]
     B, res = 4, 64
     with tempfile.TemporaryDirectory() as td:
         ck = os.path.join(td, "dino.pth")
         H.write_random_dino_checkpoint(ck, "vit_small")
         cfg = make_cfg(pretrained_weights=ck)
         batch = H.make_batch(B, res, cuda_dev)
-        runs = {}
-        for impl in ("stego_b200", "reference"):
-            ts = H.load_reference_segmenter(impl)
-            torch.manual_seed(0)
-            m = ts.LitUnsupervisedSegmenter(27, cfg).to(cuda_dev)
-            m.train()
-            torch.manual_seed(777)
-            losses = []
-            for s in range(2):
-                losses.append(float(m.training_step(batch, s).detach()))
-                m.global_step += 1
-            names = [n for n, p in m.named_parameters() if p.requires_grad]
-            runs[impl] = dict(losses=losses, logged={k: float(v) for k, v in m.logged.items()},
-                              grads={n: dict(m.named_parameters())[n].grad.detach().clone() for n in names
-                                     if dict(m.named_parameters())[n].grad is not None},
-                              params={n: dict(m.named_parameters())[n].detach().clone() for n in names})
-            if impl == "stego_b200":
-                assert type(m.net).__module__ == "stego_b200.modules"  # the class the reference text instantiated
-    ours, ref = runs["stego_b200"], runs["reference"]
-    trained = [n for n in ref["grads"] if n.startswith(("net.cluster", "linear_probe", "cluster_probe"))]
-    assert set(trained) <= set(ours["grads"])
-    errs = {n: rel(ours["grads"][n], ref["grads"][n]) for n in trained}
-    record("dropin_reference_training_step", dict(losses_ours=ours["losses"], losses_reference=ref["losses"],
-                                                   logged_ours=ours["logged"], logged_reference=ref["logged"],
-                                                   grad_rel=errs))
-    print("reference training_step text: ours", ours["losses"], "reference-eager", ref["losses"], "grad rel", errs)
-    for a, b in zip(ours["losses"], ref["losses"]):
+        torch.manual_seed(0)
+        m = LitUnsupervisedSegmenter(27, cfg).to(cuda_dev)
+    H.load_trainable_state(m, H.trainable_state())
+    m.train()
+    torch.manual_seed(777)
+    losses = [float(m.training_step(batch, s).detach()) for s in range(2)]
+    logged = {k: float(v) for k, v in m.logged.items()}
+    grads = grads_of(m)
+    errs = {n: _rel_sampled(grads[n], ref["grad"][n])[0] for n in ref["grad"]}
+    record("dropin_reference_training_step", dict(losses_ours=losses, losses_reference=ref["losses"],
+                                                   logged_ours=logged, logged_reference=ref["logged"], grad_rel=errs))
+    print("training_step: ours", losses, "reference-eager", ref["losses"], "grad rel", errs)
+    for a, b in zip(losses, ref["losses"]):
         assert abs(a - b) < 5e-3 * abs(b), (a, b)  # includes the bf16-operand backbone vs the fp32 eager backbone
     for k in ("loss/linear", "loss/cluster"):
-        assert abs(ours["logged"][k] - ref["logged"][k]) < 5e-3 * abs(ref["logged"][k]) + 1e-4
+        assert abs(logged[k] - ref["logged"][k]) < 5e-3 * abs(ref["logged"][k]) + 1e-4
     for n in ("linear_probe.weight", "linear_probe.bias", "cluster_probe.clusters"):
+        assert "idx" not in ref["grad"][n]  # stored whole
         assert errs[n] < 5e-2, (n, errs[n])

@@ -1,9 +1,7 @@
-"""CPU: the oracle against the golden fixtures produced by the REAL reference (oracle/make_golden.py),
-and against the reference itself when /root/reference is present (build container)."""
+"""CPU: the oracle against the golden fixtures produced by the REAL reference (oracle/make_golden.py)."""
 import os
 import sys
 
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -110,10 +108,27 @@ def test_clamp_gradient_is_inclusive():
     assert x.grad.tolist() == [1.0, 0.0, 1.0]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree only exists in the build container")
 def test_oracle_matches_real_reference():
-    import check_against_reference
-    assert check_against_reference.run_checks()
+    """Every check of oracle/check_against_reference.py, against the reference's outputs stored (sampled) by
+    make_golden.py: the same max|diff| bound on the stored elements, shape and norm of the whole tensor."""
+    import check_against_reference as C
+    gold = _load("reference_checks.pt")
+    got = C.oracle_outputs()
+    bad = []
+    for k, tol in C.TOL.items():
+        g, w = got[k], gold[k]
+        assert tuple(g.shape) == w["shape"], k
+        if tol is None:
+            ok = torch.equal(g.reshape(-1).to(w["val"].dtype), w["val"])
+        else:
+            flat = g.reshape(-1)
+            sub = flat[w["idx"].long()] if "idx" in w else flat
+            scale = tol * max(w["absmax"], 1.0)
+            ok = ((sub - w["val"]).abs().max().item() <= scale and
+                  abs(flat.double().norm().item() - w["norm"]) <= scale * flat.numel() ** 0.5)
+        if not ok:
+            bad.append(k)
+    assert not bad, bad
 
 
 def test_knn_oracle_against_brute_force():

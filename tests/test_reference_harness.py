@@ -1,46 +1,37 @@
 """CPU: pins the oracle's restatement of the training step (oracle/stego_oracle.py::training_losses, adam_step —
-src/train_segmentation.py:112-245, 373-383) against the REFERENCE's own LitUnsupervisedSegmenter.training_step, executed
-unmodified through the stub-Lightning harness (oracle/lightning_harness.py).  Runs only where the reference sources are
-present (baseline/_ref from __graft_entry__.build(), or /root/reference)."""
+src/train_segmentation.py:112-245, 373-383) and of the kNN helpers against what the REFERENCE's own code computed on
+the same seeded inputs: its LitUnsupervisedSegmenter.training_step executed unmodified through the stub-Lightning
+harness (oracle/lightning_harness.py), and its precompute_knns.py statements, stored by oracle/make_golden.py under
+tests/golden/."""
 import os
 import sys
-import tempfile
 
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
+GOLD = os.path.join(ROOT, "tests", "golden")
+
+
+def _sub(t, s):
+    """The elements of `t` that the stored sample `s` (make_golden.sampled) holds."""
+    flat = t.reshape(-1)
+    return flat[s["idx"].long()] if "idx" in s else flat
 
 
 def test_oracle_training_step_matches_reference_training_step():
     import lightning_harness as H
     import stego_oracle as O
-    if not H.available():
-        pytest.skip("reference sources not present")
-    from stego_b200.config import make_cfg
-    B, res, E = 2, 64, 384
-    ts = H.load_reference_segmenter("reference")
-    with tempfile.TemporaryDirectory() as td:
-        ck = os.path.join(td, "dino.pth")
-        sd = H.write_random_dino_checkpoint(ck, "vit_small")
-        cfg = make_cfg(pretrained_weights=ck)
-        torch.manual_seed(0)
-        m = ts.LitUnsupervisedSegmenter(27, cfg)
-    m.train()
-    batch = H.make_batch(B, res, "cpu")
-    names = ["net.cluster1.0.weight", "net.cluster1.0.bias", "net.cluster2.0.weight", "net.cluster2.0.bias",
-             "net.cluster2.2.weight", "net.cluster2.2.bias", "linear_probe.weight", "linear_probe.bias",
-             "cluster_probe.clusters"]
-    p0 = {k: dict(m.named_parameters())[k].detach().clone() for k in names}
-    # the draws the reference step is about to make (Dropout2d x3 for net(img), x3 for net(img_pos), rand x2, randperm x5)
+    gold = torch.load(os.path.join(GOLD, "reference_training_step.pt"))
+    B, E = 2, 384
+    sd = O.perturb_vit_state(O.vit_random_state("vit_small", 8, seed=3))  # the checkpoint the reference loaded
+    p0 = H.trainable_state()
+    batch = H.make_batch(B, 64, "cpu")
+    # the draws the reference step made (Dropout2d x3 for net(img), x3 for net(img_pos), rand x2, randperm x5)
     torch.manual_seed(777)
     masks = [O.draw_dropout2d_mask(B, E) for _ in range(3)]
     masks_pos = [O.draw_dropout2d_mask(B, E) for _ in range(3)]
     c1, c2, perms = O.draw_loss_randomness(B, O.LossCfg())
-    torch.manual_seed(777)
-    loss = m.training_step(batch, 0)
-    # oracle
     with torch.no_grad():
         f = O.vit_image_feat(sd, batch["img"], "vit_small", 8)
         fp = O.vit_image_feat(sd, batch["img_pos"], "vit_small", 8)
@@ -48,58 +39,34 @@ def test_oracle_training_step_matches_reference_training_step():
     probes = {k: v.clone().requires_grad_(True) for k, v in p0.items() if not k.startswith("net.")}
     out = O.training_losses(f, fp, hp, probes, batch["label"], masks, masks_pos, c1, c2, perms, O.LossCfg(), 27)
     out["total"].backward()
-    assert abs(float(loss) - out["total"].item()) < 2e-6 * abs(out["total"].item())
+    assert abs(gold["loss"] - out["total"].item()) < 2e-6 * abs(out["total"].item())
     for k_log, k_or in [("loss/pos_intra", "pos_intra"), ("loss/pos_inter", "pos_inter"), ("loss/neg_inter", "neg_inter"),
                         ("loss/linear", "linear"), ("loss/cluster", "cluster"), ("cd/pos_intra", "cd_intra"),
                         ("cd/pos_inter", "cd_inter"), ("cd/neg_inter", "cd_neg")]:
-        assert abs(float(m.logged[k_log]) - out[k_or].item()) < 1e-5 * abs(out[k_or].item()) + 1e-7, k_log
+        assert abs(gold["logged"][k_log] - out[k_or].item()) < 1e-5 * abs(out[k_or].item()) + 1e-7, k_log
     want_g = {("net." + k): v.grad for k, v in hp.items()}
     want_g.update({k: v.grad for k, v in probes.items()})
-    params = dict(m.named_parameters())
-    for k in names:
-        g = params[k].grad
-        assert (g - want_g[k]).norm() <= 1e-4 * want_g[k].norm() + 1e-10, k
+    for k in p0:
+        gs, ps = gold["grad"][k], gold["param"][k]
+        g, w = gs["val"], _sub(want_g[k], gs)
+        assert (g - w).norm() <= 1e-4 * w.norm() + 1e-10, k
+        assert abs(gs["norm"] - want_g[k].double().norm().item()) <= 1e-4 * want_g[k].norm().item() + 1e-10, k
         # the reference's torch.optim.Adam update vs the oracle's adam_step on the reference's gradient
-        p = p0[k].clone()
+        assert ("idx" in gs) == ("idx" in ps) and ("idx" not in gs or torch.equal(gs["idx"], ps["idx"]))
+        p = _sub(p0[k], ps).clone()
         O.adam_step(p, g, torch.zeros_like(p), torch.zeros_like(p), 1, 5e-4 if k.startswith("net.") else 5e-3)
-        assert (params[k].detach() - p).abs().max().item() < 1e-7, k
+        assert (ps["val"] - p).abs().max().item() < 1e-7, k
 
 
 def test_knn_oracle_matches_lifted_reference_lines():
     """The kNN restatement (oracle knn_descriptors / knn_indices) against the reference's own statements: `get_feats`
-    (src/precompute_knns.py:15-21) and the slab loop (:83-92), lifted as TEXT from the reference file and executed."""
-    import ast
-    import textwrap
-    import lightning_harness as H
+    (src/precompute_knns.py:15-21) and the slab loop (:83-92), lifted as TEXT from the reference file and executed by
+    make_golden.py on the same 40 descriptors."""
+    import make_golden
     import stego_oracle as O
-    src_dir = H.reference_src()
-    if src_dir is None:
-        pytest.skip("reference sources not present")
-    text = open(os.path.join(src_dir, "precompute_knns.py")).read()
-    tree = ast.parse(text)
-    get_feats_src = next(ast.get_source_segment(text, n) for n in tree.body
-                         if isinstance(n, ast.FunctionDef) and n.name == "get_feats")
-    lines = text.splitlines()
-    first = next(i for i, l in enumerate(lines) if "normed_feats = get_feats(par_model, loader)" in l)
-    last = next(i for i, l in enumerate(lines) if "nearest_neighbors = torch.cat(all_nns, dim=0)" in l)
-    loop_src = textwrap.dedent("\n".join(lines[first:last + 1]))
-    import torch.nn.functional as F
-    g = torch.Generator().manual_seed(0)
-    feats_maps = [torch.randn(8, 32, 5, 5, generator=g) for _ in range(5)]  # "model outputs" of 5 loader batches: n = 40
-    it = iter(feats_maps)
-    env = dict(torch=torch, F=F, tqdm=lambda x: x, n_batches=4)
-    orig_cuda, orig_empty = torch.Tensor.cuda, torch.cuda.empty_cache
-    torch.Tensor.cuda = lambda self, *a, **k: self  # get_feats moves the batch to the GPU; this is a CPU test
-    torch.cuda.empty_cache = lambda: None
-    try:
-        exec(get_feats_src, env)
-        env["par_model"] = type("ParModel", (), {"forward": staticmethod(lambda img: next(it))})()
-        env["loader"] = [dict(img=torch.zeros(8, 3, 4, 4)) for _ in feats_maps]
-        exec(loop_src, env)
-    finally:
-        torch.Tensor.cuda, torch.cuda.empty_cache = orig_cuda, orig_empty
-    want_feats, want_nn = env["normed_feats"], env["nearest_neighbors"]
-    desc = torch.cat([O.knn_descriptors(f) for f in feats_maps], 0)
+    gold = torch.load(os.path.join(GOLD, "reference_knn.pt"))
+    want_feats, want_nn = gold["normed_feats"], gold["nearest_neighbors"].long()
+    desc = torch.cat([O.knn_descriptors(f) for f in make_golden.knn_inputs()], 0)
     assert torch.allclose(desc, want_feats, atol=1e-7)
     idx, _ = O.knn_indices(desc, k=30, n_batches=4)
     assert idx.shape == want_nn.shape == (40, 30)

@@ -49,6 +49,12 @@ def test_multistep_graph_replay_vs_autograd_vs_oracle(cuda_dev, reset_at):
         draws = peek_draws(fused, B, cuda_dev)
         gpu_state, cpu_state = torch.cuda.get_rng_state(cuda_dev), torch.get_rng_state()
         p_before = params_of(fused)
+        # the twin starts every step from the fused model's parameters and Adam moments: left on its own trajectory it
+        # drifts from the fused one (Adam's update is sign-like for tiny gradients, and hidden activations at the ReLU /
+        # clamp kinks land on either side), which after a few steps moves hidden-layer gradients by more than the bound
+        with torch.no_grad():
+            for buf in ("param", "exp_avg", "exp_avg_sq"):
+                getattr(twin._flat, buf).copy_(getattr(fused._flat, buf))
         loss = fused.training_step(batch, s)
         g_f, p_f = grads_of(fused), params_of(fused)
         after_state = torch.cuda.get_rng_state(cuda_dev)
@@ -67,8 +73,6 @@ def test_multistep_graph_replay_vs_autograd_vs_oracle(cuda_dev, reset_at):
             # both paths run the same kernels; they differ in accumulation order (atomics) and both sit ~2e-4 from the
             # oracle on the hidden-layer weight gradient (bf16 dgrad operand), measured 3e-4 from each other
             worst["twin_grad"] = max(worst.get("twin_grad", 0.0), rel(g_f[k], g_t[k]))
-            # (the twin follows its OWN parameter trajectory, ~1e-6 away after a few steps: hidden activations that sit at
-            # the ReLU / clamp kinks land on either side, so the hidden-layer gradients of the two runs drift to ~1e-3)
             assert rel(g_f[k], g_t[k]) < 3e-3, (s, k, rel(g_f[k], g_t[k]))
             worst["twin_param"] = max(worst["twin_param"], rel(p_f[k], p_t[k]))
             assert rel(p_f[k], p_t[k]) < 2e-4, (s, k, rel(p_f[k], p_t[k]))
